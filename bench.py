@@ -73,9 +73,11 @@ while True:
     try:
         sm = nv.nvmlDeviceGetClockInfo(h, nv.NVML_CLOCK_SM)
         r = nv.nvmlDeviceGetCurrentClocksThrottleReasons(h)
-        out.write('%.6f %d %d %d\n' % (time.time(), sm, mx, r)); out.flush()
     except Exception:
-        pass
+        sm = None
+    if sm is not None:
+        # raises once bench.py is gone (its end of the pipe closes), which ends the poller with it
+        out.write('%.6f %d %d %d\n' % (time.time(), sm, mx, r)); out.flush()
     time.sleep(0.002)
 """
 
@@ -341,7 +343,7 @@ def mapping_record(args, synth, pkg, ctx_feat, rank, world, local_rank, dist, to
     """BASELINE configs[2] / [3]: scan-to-map against a 1M-point-per-GPU voxel map (N > 1: sharded, real ncclAllReduce)."""
     shard = importlib.import_module("a-loam_b200.shard")
     total_pts = 1_000_000 * world
-    Km = min(K, len(synth.MAP_QUERY_SCANS) - 3)
+    Km = K
     Wm = 3
 
     def feats(raw):
@@ -391,7 +393,9 @@ def mapping_record(args, synth, pkg, ctx_feat, rank, world, local_rank, dist, to
             l0 = ctx.launch_count()
             t0 = time.perf_counter()
             ctx.map_upload_ptr(mc.data_ptr(), mc.shape[0], ms.data_ptr(), ms.shape[0])
-            x, st = ctx.mapping_register(stacks[i][0], stacks[i][1], stacks[i][2])
+            # past the last query scan the stacks repeat: a step re-uploads and re-indexes the map after an L2 flush either way
+            cs, ss, x0, _k = stacks[i % len(stacks)]
+            x, st = ctx.mapping_register(cs, ss, x0)
             t1 = time.perf_counter()
             if i >= Wm:
                 step_s.append(t1 - t0); poses.append(x); launches += ctx.launch_count() - l0
@@ -613,6 +617,18 @@ def batch_record(args, synth, pkg, rank, world, local_rank, dist, torch, K, W):
     return rec
 
 
+def dump_outputs(out_dir, poses, stats):
+    """what the caller of the headline path receives from its last timed aloam_scan_stream call (K device-resident scans):
+    poses.npy (K, 7) float64 world poses (q xyzw, t), and stats_last.npy float64 [n_corner_corr, n_plane_corr, lm_iters,
+    accepted_steps, flags, termination[4], init_cost, final_cost] of its last scan (ms_total, a time, is left out)"""
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "poses.npy"), np.ascontiguousarray(poses, np.float64))
+    d = stats.as_dict()
+    np.save(os.path.join(out_dir, "stats_last.npy"), np.array(
+        [d["n_corner_corr"], d["n_plane_corr"], d["lm_iters"], d["accepted_steps"], d["flags"]] + d["termination"] + [d["init_cost"], d["final_cost"]],
+        np.float64))
+
+
 def emit(line):
     sys.stdout.flush()
     os.write(_REAL_STDOUT, (json.dumps(line) + "\n").encode())
@@ -632,8 +648,14 @@ def main():
     ap.add_argument("--no-mapping", action="store_true", help="skip the scan-to-map sub-record (configs[2] / [3])")
     ap.add_argument("--no-batch", action="store_true", help="skip the batched-stream sub-record (configs[4])")
     ap.add_argument("--no-mapped", action="store_true", help="skip the full three-stage stream (odometry + map cube store)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last timed aloam_scan_stream call "
+                    "returned as DIR/poses.npy and DIR/stats_last.npy (the inputs are seeded: same arguments, same inputs)")
     args = ap.parse_args()
-    K, W = max(args.steps, 1), max(args.warmup, 3)   # never fewer than 3 untimed warm-up steps
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl ours)")
+    K, W = args.steps, max(args.warmup, 3)   # never fewer than 3 untimed warm-up steps
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -732,7 +754,7 @@ def main():
             barrier()
             secs.append(t1 - t0); devms.append(st.ms_total); launches = ctx.launch_count() - l0
             poses_all.append(poses)
-        return secs, devms, launches, np.concatenate(poses_all)
+        return secs, devms, launches, np.concatenate(poses_all), st
 
     def run_sync(mode, profile=False):
         """one synchronous aloam_scan_to_pose(_device) call per scan (latency mode); profiling covers the timed steps only"""
@@ -759,8 +781,8 @@ def main():
         return t1 - t0, dev_ms, np.concatenate([q, t])
 
     sampler.start()
-    secs_dev, devms_dev, launches, poses_dev = run_stream("device")
-    secs_e2e, _, _, poses_e2e = run_stream("host")
+    secs_dev, devms_dev, launches, poses_dev, stats_dev = run_stream("device")
+    secs_e2e, _, _, poses_e2e, _ = run_stream("host")
     sync_dev, devms_sync, pose_sync = run_sync("device")
     sync_e2e, _, _ = run_sync("host")
     clocks = sampler.stop()
@@ -855,6 +877,8 @@ def main():
                                "device_vs_host_path_identical": bool(np.array_equal(poses_dev, poses_e2e)),
                                "t_w_stream_vs_sync_maxabs": float(np.abs(poses_dev[W + K, 4:] - pose_sync[4:]).max())},
                 "mapping": mapping, "batch": batch, "mapped_stream": mapped}
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, poses_dev[-K:], stats_dev)
         emit(line)
     ctx.close()
     if world > 1:

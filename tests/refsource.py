@@ -1,30 +1,70 @@
-"""Helpers shared by tests/test_oracle_vs_reference_source.py (CPU) and tests/test_gpu_vs_reference_source.py (GPU): load the
-libraries of oracle/_ref -- the reference's own translation units compiled unmodified against the stand-in headers of
-oracle/ref_shim -- and drive them from Python.  TEST INFRASTRUCTURE."""
+"""Helpers shared by tests/test_oracle_vs_reference_source.py (CPU), tests/test_gpu_vs_reference_source.py (GPU) and
+tests/golden/make_reference_golden.py.  TEST INFRASTRUCTURE.
+
+The tests compare with tests/golden/reference_source.npz: what the libraries of oracle/_ref -- the reference's own translation
+units compiled unmodified against the stand-in headers of oracle/ref_shim -- computed on the tests' inputs.  The classes below
+load and drive those libraries from Python; only the golden generator uses them, so the tests run wherever the repository does.
+Small results (poses, counts, Jacobians) are stored as they are; clouds and work arrays as `digest`s."""
 import ctypes as C
+import hashlib
 import os
 import shutil
-import subprocess
 import tempfile
 
 import numpy as np
-import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 REF_DIR = os.path.join(ROOT, "oracle", "_ref")
+GOLDEN = os.path.join(ROOT, "tests", "golden", "reference_source.npz")
 NCUBE = 21 * 21 * 11
 TOPICS = {"full": "/velodyne_cloud_2", "sharp": "/laser_cloud_sharp", "less_sharp": "/laser_cloud_less_sharp",
           "flat": "/laser_cloud_flat", "less_flat": "/laser_cloud_less_flat"}
+CLOUDS = ("full", "sharp", "less_sharp", "flat", "less_flat")
+
+
+def digest(a):
+    """dtype, shape and SHA-256 of the bytes: two arrays have the same digest exactly when they are equal bit for bit, so a
+    bit-exact comparison with a cloud of ~100k points needs 100 bytes of golden data instead of 1.6 MB"""
+    a = np.ascontiguousarray(a)
+    return "%s %s %s" % (a.dtype.str, "x".join(str(d) for d in a.shape), hashlib.sha256(a.tobytes()).hexdigest())
+
+
+def cube_store_digest(cubes):
+    """one digest over the non-empty cubes of a store in index order (with the per-cube sizes equal, the same digest means
+    every cube is equal bit for bit)"""
+    return digest(np.concatenate(cubes) if cubes else np.zeros((0, 4), np.float32))
+
+
+_GOLDEN = None
+
+
+def golden():
+    """tests/golden/reference_source.npz as a dict: key -> array, or key -> digest string (stored together as `digests`)"""
+    global _GOLDEN
+    if _GOLDEN is None:
+        with np.load(GOLDEN, allow_pickle=False) as z:
+            _GOLDEN = {k: z[k] for k in z.files if k != "digests"}
+            _GOLDEN.update((k.decode(), v.decode()) for k, v in z["digests"])
+    return _GOLDEN
+
+
+def assert_digest(key, a, *msg):
+    assert digest(a) == golden()[key], (key,) + msg
+
+
+def assert_clouds(key, f, raw=None):
+    """the five clouds of oracle Features `f` are bit-identical to what the reference's laserCloudHandler published under `key`"""
+    if raw is not None:
+        assert_digest(key + "/raw", raw, "not the scan the golden data was recorded on")
+    for name in CLOUDS:
+        assert_digest("%s/%s" % (key, name), getattr(f, name))
 
 
 def ref_lib(name):
-    """builds oracle/_ref/<name> where /root/reference exists, uses the prebuilt file elsewhere, skips the test if there is none"""
-    if os.path.isdir("/root/reference/src"):
-        r = subprocess.run(["make", "-C", os.path.join(ROOT, "oracle"), "_ref/" + name], capture_output=True, text=True)
-        assert r.returncode == 0, r.stdout + r.stderr
+    """oracle/_ref/<name>: built by `make -C oracle ref REF=<checkout of the reference>` (build() does it where the sources are)"""
     path = os.path.join(REF_DIR, name)
     if not os.path.exists(path):
-        pytest.skip("oracle/_ref/%s is not built and /root/reference is not present" % name)
+        raise FileNotFoundError("oracle/_ref/%s is not built: run `make -C oracle ref REF=<checkout of the reference>`" % name)
     return C.CDLL(path)
 
 
