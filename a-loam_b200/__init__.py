@@ -15,6 +15,8 @@ _LIB = None
 
 OK = 0
 FLAG_FEW_CORRESPONDENCES, FLAG_MAP_TOO_THIN, FLAG_INITIALISED_ONLY, FLAG_CUBE_OVERFLOW = 1, 2, 4, 8
+FLAG_OUTPUT_TRUNCATED = 16
+MAP_SURROUND, MAP_ALL = 0, 1
 BLOCK_DOUBLES = 11
 
 EXPORTED_SYMBOLS = [
@@ -23,6 +25,7 @@ EXPORTED_SYMBOLS = [
     "aloam_voxel_filter", "aloam_scan_to_pose", "aloam_scan_to_pose_device", "aloam_reset_odometry", "aloam_knn",
     "aloam_odometry_associate", "aloam_normal_equations", "aloam_solve", "aloam_debug_features", "aloam_mapping_associate",
     "aloam_comm_unique_id", "aloam_comm_init", "aloam_comm_uses_peer_memory", "aloam_map_upload_sharded", "aloam_scan_stream", "aloam_scan_stream_batch", "aloam_scan_stream_mapped", "aloam_transform_to_end", "aloam_mapper_reset", "aloam_mapper_step", "aloam_profile_enable", "aloam_profile_read", "aloam_launch_count",
+    "aloam_mapper_export", "aloam_mapper_associate_to_map", "aloam_scan_stream_mapped_registered",
 ]
 
 
@@ -85,6 +88,10 @@ def lib():
         L.aloam_mapper_step.argtypes = [C.c_void_p, cv, cv, dp, dp, dp, dp, C.POINTER(Stats)]
         L.aloam_mapper_debug_state.argtypes = [C.c_void_p, ip, ip, ip, dp, dp, C.POINTER(C.c_longlong)]
         L.aloam_mapper_debug_cube.argtypes = [C.c_void_p, C.c_int, C.c_int, C.POINTER(cv)]
+        L.aloam_mapper_export.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_longlong, C.POINTER(C.c_longlong)]
+        L.aloam_mapper_associate_to_map.argtypes = [C.c_void_p, cv, C.c_void_p]
+        L.aloam_scan_stream_mapped_registered.argtypes = [C.c_void_p, C.POINTER(cv), C.c_int, C.c_int, dp, dp, C.c_void_p, C.c_longlong,
+                                                          C.POINTER(C.c_longlong), C.POINTER(Stats)]
         L.aloam_scan_to_pose.argtypes = [C.c_void_p, cv, dp, dp, C.POINTER(Stats)]
         L.aloam_scan_to_pose_device.argtypes = [C.c_void_p, C.c_void_p, C.c_int, dp, dp, C.POINTER(Stats)]
         L.aloam_reset_odometry.argtypes = [C.c_void_p]
@@ -253,6 +260,44 @@ class Aloam:
         out = CloudView()
         _check(lib().aloam_mapper_debug_cube(self._h, which, cube_index, C.byref(out)))
         return _out(out)
+
+    # --- map outputs (laserMapping.cpp:803-848)
+    def mapper_export_ptr(self, region, ptr, capacity):
+        """aloam_mapper_export into caller memory at `ptr` (host or device address, room for `capacity` points); returns the
+        number of points.  ptr = 0 with capacity = 0 only asks for the size."""
+        n = C.c_longlong(0)
+        _check(lib().aloam_mapper_export(self._h, int(region), C.c_void_p(int(ptr)) if ptr else None, int(capacity), C.byref(n)))
+        return n.value
+
+    def mapper_export(self, region):
+        """/laser_cloud_surround (MAP_SURROUND) or /laser_cloud_map (MAP_ALL) as an (n, 4) float32 array"""
+        n = self.mapper_export_ptr(region, 0, 0)
+        out = np.zeros((n, 4), np.float32)
+        if n:
+            self.mapper_export_ptr(region, out.ctypes.data, n)
+        return out
+
+    def mapper_associate_to_map(self, cloud):
+        """/velodyne_cloud_registered: pointAssociateToMap of `cloud` with the refined pose of the last frame -> (n, 4)"""
+        v, keep = _view(cloud)
+        out = np.zeros((v.n, 4), np.float32)
+        _check(lib().aloam_mapper_associate_to_map(self._h, v, out.ctypes.data if v.n else None))
+        return out
+
+    def scan_stream_mapped_registered(self, ptrs, counts, device_resident, out_ptr, capacity, stride=4):
+        """scan_stream_mapped, and every scan's registered full cloud written to out_ptr (device or pinned host address,
+        room for `capacity` points) at offsets[k]; returns (odom poses, map poses, offsets (n + 1), stats dict)"""
+        n = len(ptrs)
+        views = (CloudView * n)()
+        for i in range(n):
+            views[i] = CloudView(C.cast(C.c_void_p(int(ptrs[i])), C.POINTER(C.c_float)), int(counts[i]), stride)
+        odom = np.zeros((n, 7)); mapped = np.zeros((n, 7))
+        offsets = np.zeros(n + 1, np.int64)
+        st = Stats()
+        _check(lib().aloam_scan_stream_mapped_registered(self._h, views, n, int(device_resident), _dp(odom), _dp(mapped),
+                                                         C.c_void_p(int(out_ptr)) if out_ptr else None, int(capacity),
+                                                         offsets.ctypes.data_as(C.POINTER(C.c_longlong)), C.byref(st)))
+        return odom, mapped, offsets, st.as_dict()
 
     def mapping_register(self, corner_stack, surf_stack, x):
         a, ka = _view(corner_stack)

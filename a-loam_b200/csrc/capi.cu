@@ -80,6 +80,12 @@ int aloam_destroy(aloam_ctx* c) {
   for (cudaEvent_t e : c->ev_mapdone) if (e) cudaEventDestroy(e);
   for (cudaEvent_t e : c->ev_h2d) if (e) cudaEventDestroy(e);
   for (cudaEvent_t e : c->ev_rawfree) if (e) cudaEventDestroy(e);
+  if (c->s_reg) { cudaStreamSynchronize(c->s_reg); cudaStreamDestroy(c->s_reg); }
+  for (cudaEvent_t e : c->ev_regcopy) if (e) cudaEventDestroy(e);
+  for (cudaEvent_t e : c->ev_regdone) if (e) cudaEventDestroy(e);
+  for (cudaEvent_t e : c->ev_fullfree) if (e) cudaEventDestroy(e);
+  for (Pt4* p : c->d_reg_full) if (p) cudaFree(p);
+  if (c->d_reg_off) cudaFree(c->d_reg_off);
   if (c->h_poses) cudaFreeHost(c->h_poses);
   if (c->h_scan_nfull) cudaFreeHost(c->h_scan_nfull);
   for (Lane& L : c->lanes) free_lane(L);
@@ -322,7 +328,7 @@ struct StreamGuard {
 };
 
 void sync_all_streams(aloam_ctx* c) {
-  cudaStream_t ss[] = {c->stream, c->s_ext, c->s_exa, c->s_idx, c->s_h2d, c->s_map};
+  cudaStream_t ss[] = {c->stream, c->s_ext, c->s_exa, c->s_idx, c->s_h2d, c->s_map, c->s_reg};
   for (cudaStream_t s : ss) if (s) cudaStreamSynchronize(s);
 }
 
@@ -542,14 +548,45 @@ int aloam_scan_to_pose_device(aloam_ctx* c, const float* d_raw, int n, double q_
   return scan_to_pose_impl(c, d_raw, n, 4, q_w, t_w, stats);
 }
 
+// registered full-resolution clouds of aloam_scan_stream_mapped_registered
+struct RegisteredOut {
+  float* points;         // device or page-locked host memory
+  long long capacity;    // in points
+  long long* offsets;    // [n_scans + 1], host
+};
+
+// the stream buffers of the registered clouds, created on first use (contexts that never ask for them do not grow)
+static int ensure_registered_buffers(aloam_ctx* c) {
+  if (c->s_reg) return ALOAM_OK;
+  bool ok = dalloc(&c->d_reg_off, (size_t)kMaxStreamScans + 1) == cudaSuccess;
+  for (Pt4*& p : c->d_reg_full) ok = ok && dalloc(&p, (size_t)c->max_points) == cudaSuccess;
+  for (cudaEvent_t& e : c->ev_regcopy) ok = ok && cudaEventCreateWithFlags(&e, cudaEventDisableTiming) == cudaSuccess;
+  for (cudaEvent_t& e : c->ev_regdone) ok = ok && cudaEventCreateWithFlags(&e, cudaEventDisableTiming) == cudaSuccess;
+  for (cudaEvent_t& e : c->ev_fullfree) ok = ok && cudaEventCreateWithFlags(&e, cudaEventDisableTiming) == cudaSuccess;
+  ok = ok && cudaStreamCreateWithFlags(&c->s_reg, cudaStreamNonBlocking) == cudaSuccess;
+  if (!ok) {   // keep nothing half-built: the next call tries again
+    cudaGetLastError();
+    if (c->s_reg) cudaStreamDestroy(c->s_reg);
+    c->s_reg = nullptr;
+    for (cudaEvent_t* es : {c->ev_regcopy, c->ev_regdone}) for (int i = 0; i < kFeatSlots; ++i) { if (es[i]) cudaEventDestroy(es[i]); es[i] = nullptr; }
+    for (cudaEvent_t& e : c->ev_fullfree) { if (e) cudaEventDestroy(e); e = nullptr; }
+    for (Pt4*& p : c->d_reg_full) { if (p) cudaFree(p); p = nullptr; }
+    if (c->d_reg_off) cudaFree(c->d_reg_off);
+    c->d_reg_off = nullptr;
+    return ALOAM_ERR_CUDA;
+  }
+  return ALOAM_OK;
+}
+
 // Pipelined form of aloam_scan_to_pose for a sequence of scans of `nb` trajectories in lockstep: ring binning of scan k+1
 // (s_exa), per-ring extraction (s_ext), compaction + index build (s_idx) run concurrently with association + LM of scan k
 // (main stream) and the host->device copies of scan k+2 (s_h2d) -- the overlap the reference gets from its three ROS
 // processes.  Every launch covers all nb trajectories.  Results are identical to calling aloam_scan_to_pose once per scan
 // and trajectory.  raws / poses are scan-major: entry k * nb + b.
 static int scan_stream_impl(aloam_ctx* c, const aloam_cloud_view* raws, int n_scans, int nb, int device_resident, double* poses, aloam_stats* stats_last,
-                            double* map_poses = nullptr) {
+                            double* map_poses = nullptr, const RegisteredOut* reg = nullptr) {
   if (map_poses && (nb != 1 || !c || c->cfg.max_map_points <= 0)) return ALOAM_ERR_INVALID_ARG;
+  if (reg && (!map_poses || !reg->points || !reg->offsets || reg->capacity < 0)) return ALOAM_ERR_INVALID_ARG;
   if (!c || !raws || !poses || n_scans < 1 || nb < 1 || nb > c->n_lanes || (long long)n_scans * nb > kMaxStreamScans) return ALOAM_ERR_INVALID_ARG;
   for (int k = 0; k < n_scans * nb; ++k) {
     int rc = check_view(raws[k]); if (rc) return rc;
@@ -559,6 +596,16 @@ static int scan_stream_impl(aloam_ctx* c, const aloam_cloud_view* raws, int n_sc
     if (raws[k].stride_floats != raws[k - k % nb].stride_floats) return ALOAM_ERR_INVALID_ARG;   // one stride per step
   }
   CUDA_CHECK_RET(cudaSetDevice(c->cfg.device));
+  Pt4* reg_out = nullptr;
+  if (reg) {
+    // the clouds are written by a kernel: device memory of this context's GPU, or page-locked host memory it can address
+    cudaPointerAttributes pa;
+    if (cudaPointerGetAttributes(&pa, reg->points) != cudaSuccess) { cudaGetLastError(); return ALOAM_ERR_INVALID_ARG; }
+    const bool dev = (pa.type == cudaMemoryTypeDevice || pa.type == cudaMemoryTypeManaged) && pa.device == c->cfg.device;
+    if (!(dev || pa.type == cudaMemoryTypeHost) || !pa.devicePointer) return ALOAM_ERR_INVALID_ARG;
+    reg_out = static_cast<Pt4*>(pa.devicePointer);
+    int rc = ensure_registered_buffers(c); if (rc) return rc;
+  }
   if (map_poses && !c->mapper) { int rc = aloam_mapper_reset(c); if (rc) return rc; }   // creates the cube store
   StreamGuard guard(c);
   cudaStream_t s_main = c->stream;
@@ -579,6 +626,7 @@ static int scan_stream_impl(aloam_ctx* c, const aloam_cloud_view* raws, int n_sc
   // Waiting on an event that was never recorded, or whose work finished in an earlier call, is a no-op -- so the
   // per-scan waits below need no "first iterations" special cases.
   for (cudaStream_t s : {c->s_h2d, c->s_exa, c->s_ext, c->s_idx, c->s_map}) STREAM_TRY(cudaStreamWaitEvent(s, c->ev0, 0));
+  if (reg) STREAM_TRY(cudaStreamWaitEvent(c->s_reg, c->ev0, 0));
   const float* d_raw[ALOAM_MAX_BATCH];
   int ns[ALOAM_MAX_BATCH];
   for (int k = 0; k < n_scans; ++k) {
@@ -601,6 +649,7 @@ static int scan_stream_impl(aloam_ctx* c, const aloam_cloud_view* raws, int n_sc
     }
     // ---- stage A (ring binning) on s_exa: needs full[b] free, i.e. stage B of scan k-2 done
     STREAM_TRY(cudaStreamWaitEvent(c->s_exa, c->ev_b[b], 0));
+    if (reg) STREAM_TRY(cudaStreamWaitEvent(c->s_exa, c->ev_fullfree[b], 0));   // stage C of scan k-2 has copied full[b] out
     c->stream = c->s_exa;
     int sc_slot = 0;
     int rc = run_features_a(c, nb, d_raw, ns, device_resident ? 4 : rv[0].stride_floats, b, &sc_slot, c->d_scan_nfull + (size_t)k * nb);
@@ -628,6 +677,14 @@ static int scan_stream_impl(aloam_ctx* c, const aloam_cloud_view* raws, int n_sc
     STREAM_TRY(cudaEventRecord(c->ev_feat[cur], c->s_idx));
     run_grid_build(c, nb, cur, 64 * kMaxLessSharpPerRing, std::min(nmax, c->max_points));
     STREAM_TRY(cudaEventRecord(c->ev_idx[cur], c->s_idx));
+    if (reg) {
+      // the ring-major cloud outlives full[b] (stage A of scan k+2 overwrites it) in slot `cur`, free once the registered cloud
+      // of frame f - kFeatSlots has been written
+      STREAM_TRY(cudaStreamWaitEvent(c->s_idx, c->ev_regdone[cur], 0));
+      map_out_stage_full(c, c->lanes[0].d_full[b], c->d_scan_nfull + k, nmax, k, c->d_reg_full[cur], c->d_reg_off);
+      STREAM_TRY(cudaEventRecord(c->ev_fullfree[b], c->s_idx));
+      STREAM_TRY(cudaEventRecord(c->ev_regcopy[cur], c->s_idx));
+    }
     c->stream = s_main;
     // ---- association + LM on the main stream: this scan's sharp / flat points, the previous scan's clouds + index
     STREAM_TRY(cudaStreamWaitEvent(s_main, c->ev_feat[cur], 0));
@@ -648,6 +705,14 @@ static int scan_stream_impl(aloam_ctx* c, const aloam_cloud_view* raws, int n_sc
                               c->d_poses + (size_t)k * 7, c->d_map_poses + (size_t)k * 7);
       if (rc) return fail(rc);
       STREAM_TRY(cudaEventRecord(c->ev_mapdone[cur], c->s_map));
+      if (reg) {
+        // /velodyne_cloud_registered (laserMapping.cpp:838-848) with this frame's refined pose, beside the next frames' mapping
+        STREAM_TRY(cudaStreamWaitEvent(c->s_reg, c->ev_mapdone[cur], 0));
+        STREAM_TRY(cudaStreamWaitEvent(c->s_reg, c->ev_regcopy[cur], 0));
+        c->stream = c->s_reg;
+        map_out_register(c, c->d_reg_full[cur], c->d_scan_nfull + k, nmax, c->d_reg_off + k, reg->capacity, c->d_map_poses + (size_t)k * 7, reg_out);
+        STREAM_TRY(cudaEventRecord(c->ev_regdone[cur], c->s_reg));
+      }
       c->stream = s_main;
     }
     c->cur = cur;
@@ -688,6 +753,11 @@ static int scan_stream_impl(aloam_ctx* c, const aloam_cloud_view* raws, int n_sc
       else fill_stats_from(c->h_summary + 4 * l, &stats_last[l], c->cfg.outer_iters, 0, ms);
     }
   }
+  if (reg) {   // the same prefix sum the device ran; scans that end beyond the capacity were not written
+    reg->offsets[0] = 0;
+    for (int k = 0; k < n_scans; ++k) reg->offsets[k + 1] = reg->offsets[k] + c->h_scan_nfull[k];
+    if (reg->offsets[n_scans] > reg->capacity && stats_last) stats_last->flags |= ALOAM_FLAG_OUTPUT_TRUNCATED;
+  }
   return ALOAM_OK;
 }
 
@@ -699,6 +769,13 @@ int aloam_scan_stream_mapped(aloam_ctx* c, const aloam_cloud_view* raws, int n_s
                              aloam_stats* stats_last) {
   if (!map_poses) return ALOAM_ERR_INVALID_ARG;
   return scan_stream_impl(c, raws, n_scans, 1, device_resident, odom_poses, stats_last, map_poses);
+}
+
+int aloam_scan_stream_mapped_registered(aloam_ctx* c, const aloam_cloud_view* raws, int n_scans, int device_resident, double* odom_poses, double* map_poses,
+                                        float* registered, long long capacity_points, long long* offsets, aloam_stats* stats_last) {
+  if (!map_poses) return ALOAM_ERR_INVALID_ARG;
+  const RegisteredOut reg{registered, capacity_points, offsets};
+  return scan_stream_impl(c, raws, n_scans, 1, device_resident, odom_poses, stats_last, map_poses, &reg);
 }
 
 int aloam_scan_stream_batch(aloam_ctx* c, const aloam_cloud_view* raws, int n_scans, int batch, int device_resident, double* poses,

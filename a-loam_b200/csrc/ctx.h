@@ -99,6 +99,13 @@ struct aloam_ctx {
   double* d_poses = nullptr;     // device [kMaxStreamScans][7]: per-(scan, lane) world poses of a stream call (one D2H at the end)
   double* d_map_poses = nullptr; // device [kMaxStreamScans][7]: map-refined poses (aloam_scan_stream_mapped)
   int* h_scan_nfull = nullptr;   // pinned [kMaxStreamScans]
+  // aloam_scan_stream_mapped_registered, created on its first call: every scan's ring-major cloud is copied out of the
+  // double-buffered d_full into a per-feature-slot buffer in stage C, then put through pointAssociateToMap with the scan's
+  // refined pose on s_reg, behind that scan's mapping step (the s_map chain is not lengthened)
+  Pt4* d_reg_full[kFeatSlots] = {};
+  long long* d_reg_off = nullptr;   // [kMaxStreamScans + 1] running prefix of the cloud sizes of the current call
+  cudaStream_t s_reg = nullptr;
+  cudaEvent_t ev_regcopy[kFeatSlots] = {}, ev_regdone[kFeatSlots] = {}, ev_fullfree[2] = {};
   // pinned host mirrors
   Pt4* h_out[5] = {nullptr, nullptr, nullptr, nullptr, nullptr};
   Pt4* h_vox_out = nullptr;     // result of aloam_voxel_filter (never aliases the feature views)
@@ -125,10 +132,11 @@ struct aloam_ctx {
 namespace {
 
 enum { KID_CLASSIFY = 0, KID_RING_SCAN, KID_SCATTER, KID_RING_FEATURES, KID_COMPACT, KID_GRID_BUILD, KID_ODOM_ASSOC, KID_LM_SOLVE,
-       KID_RING_OFFSETS, KID_KNN_LAST, KID_PACK_BLOCKS, KID_MAP_GRID, KID_MAP_KNN5, KID_VOXEL, KID_MAP_KNN, KID_MAP_FIT, KID_CUBES, KID_LM_SHARD };
+       KID_RING_OFFSETS, KID_KNN_LAST, KID_PACK_BLOCKS, KID_MAP_GRID, KID_MAP_KNN5, KID_VOXEL, KID_MAP_KNN, KID_MAP_FIT, KID_CUBES, KID_LM_SHARD,
+       KID_MAP_OUTPUT };
 const char* const kKernelNames[ALOAM_N_KERNEL_IDS] = {"k_classify", "k_ring_scan", "k_scatter", "k_ring_features", "k_compact",
     "k_rab_build(3 launches)", "k_odom_assoc", "k_lm_solve", "k_ring_offsets", "k_knn_last", "k_pack_blocks", "k_map_grid(4 launches)", "k_map_knn5",
-    "k_voxel", "k_map_knn", "k_map_fit", "k_cube_store", "k_lm_shard"};
+    "k_voxel", "k_map_knn", "k_map_fit", "k_cube_store", "k_lm_shard", "k_map_outputs"};
 
 inline void prof_begin(aloam_ctx* c, int kid) {
   ++c->launches;
@@ -195,6 +203,11 @@ int vox_seg_alloc(aloam::SegBuffers& b, size_t cap);
 void vox_seg_free(aloam::SegBuffers& b);
 int mapper_step_device(aloam_ctx* c, const Pt4* d_corner_last, const int* d_nc, int n_upper_c, const Pt4* d_surf_last, const int* d_ns, int n_upper_s,
                        const double* d_odom7, double* d_out7);
+// map outputs (cubemap.cu), on c->stream.  Stage C of the registered stream: copy scan k's ring-major cloud (size *d_n) to
+// dst and advance the running offsets off[k + 1] = off[k] + *d_n.  Then, behind the scan's mapping step: pointAssociateToMap
+// of those points with pose x7 into out[off[k] ...] when off[k + 1] <= capacity (n_upper bounds *d_n).
+void map_out_stage_full(aloam_ctx* c, const Pt4* full, const int* d_n, int n_upper, int k, Pt4* dst, long long* off);
+void map_out_register(aloam_ctx* c, const Pt4* src, const int* d_n, int n_upper, const long long* off_k, long long capacity, const double* x7, Pt4* out);
 void map_index_build(aloam_ctx* c, const Pt4* d_corner, const Pt4* d_surf, int n_upper);
 int map_shard_index_device(aloam_ctx* c, const Pt4* sub_corner, const int* n_corner, const Pt4* sub_surf, const int* n_surf, int n_upper, int* err_word);
 void map_register_device(aloam_ctx* c, const Pt4* d_corner_stack, const Pt4* d_surf_stack, const int* d_counts3, int nq_upper, double* d_pose, bool want_fits);

@@ -74,6 +74,10 @@ struct Mapper {
   int max_sub = 0;
   cudaStream_t s_aux = nullptr;             // the stack filters run here, beside the submap gather + index build
   cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
+  int* d_seg_off = nullptr;                 // [2 * NCUBE + 1] aloam_mapper_export: segment offsets, then the total
+  Pt4* d_export = nullptr;                  // aloam_mapper_export to host memory: grow-only staging
+  size_t export_cap = 0;
+  bool stepped = false;                     // a frame has run since the last reset (MapperState::x is a refined pose)
 };
 
 // ---- Eigen-order quaternion helpers (operation order of Eigen::Quaternion: the pose hand-off is compared bit for bit)
@@ -263,7 +267,26 @@ __global__ void k_mapper_update(MapperState* S, double* __restrict__ out7) {
   S->frames++;
 }
 
-// pointAssociateToMap (:154-163) in double, stored as float, then the cube of the stored point (:741-758)
+// parameters[7] (q_w_curr x, y, z, w ; t_w_curr) in registers
+struct PoseD { double ux, uy, uz, w, tx, ty, tz; };
+__device__ __forceinline__ PoseD load_pose(const double* x) { return PoseD{x[0], x[1], x[2], x[3], x[4], x[5], x[6]}; }
+
+// pointAssociateToMap (:154-163): q_w_curr * p + t_w_curr in double, in Eigen's operation order (this file is compiled with
+// -fmad=false: the bit parity with the reference depends on it), stored as float; the intensity is kept
+__device__ __forceinline__ Pt4 point_associate_to_map(const Pt4& p, const PoseD& P) {
+  const double vx = (double)p.x, vy = (double)p.y, vz = (double)p.z;
+  double uvx = P.uy * vz - P.uz * vy, uvy = P.uz * vx - P.ux * vz, uvz = P.ux * vy - P.uy * vx;
+  uvx = uvx + uvx; uvy = uvy + uvy; uvz = uvz + uvz;
+  const double cx = P.uy * uvz - P.uz * uvy, cy = P.uz * uvx - P.ux * uvz, cz = P.ux * uvy - P.uy * uvx;
+  Pt4 s;
+  s.x = (float)(((vx + P.w * uvx) + cx) + P.tx);
+  s.y = (float)(((vy + P.w * uvy) + cy) + P.ty);
+  s.z = (float)(((vz + P.w * uvz) + cz) + P.tz);
+  s.i = p.i;
+  return s;
+}
+
+// pointAssociateToMap, then the cube of the stored point (:741-758)
 // blockIdx.y = cloud (0 corner stack, 1 surf stack); the scratch of cloud 1 starts `scratch_stride` elements in
 __global__ void k_cube_ids(const Pt4* __restrict__ stack0, const Pt4* __restrict__ stack1, const MapperState* __restrict__ S, Pt4* __restrict__ world,
                            int* __restrict__ cube, int scratch_stride) {
@@ -273,19 +296,10 @@ __global__ void k_cube_ids(const Pt4* __restrict__ stack0, const Pt4* __restrict
   const Pt4* __restrict__ stack = which ? stack1 : stack0;
   world += (size_t)which * scratch_stride; cube += (size_t)which * scratch_stride;
   const int n = S->stack_counts[which];
-  const double ux = S->x[0], uy = S->x[1], uz = S->x[2], w = S->x[3], tx = S->x[4], ty = S->x[5], tz = S->x[6];
+  const PoseD P = load_pose(S->x);
   const int c0 = S->cen[0], c1 = S->cen[1], c2 = S->cen[2];
   for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
-    const Pt4 p = stack[i];
-    const double vx = (double)p.x, vy = (double)p.y, vz = (double)p.z;
-    double uvx = uy * vz - uz * vy, uvy = uz * vx - ux * vz, uvz = ux * vy - uy * vx;
-    uvx = uvx + uvx; uvy = uvy + uvy; uvz = uvz + uvz;
-    const double cx = uy * uvz - uz * uvy, cy = uz * uvx - ux * uvz, cz = ux * uvy - uy * uvx;
-    Pt4 s;
-    s.x = (float)(((vx + w * uvx) + cx) + tx);
-    s.y = (float)(((vy + w * uvy) + cy) + ty);
-    s.z = (float)(((vz + w * uvz) + cz) + tz);
-    s.i = p.i;
+    const Pt4 s = point_associate_to_map(stack[i], P);
     const int ci = cube_coord((double)s.x, c0), cj = cube_coord((double)s.y, c1), ck = cube_coord((double)s.z, c2);
     world[i] = s;
     cube[i] = (ci >= 0 && ci < CW && cj >= 0 && cj < CH && ck >= 0 && ck < CD) ? cube_index(ci, cj, ck) : -1;
@@ -362,6 +376,82 @@ __global__ void __launch_bounds__(256) k_seg_cubes(MapperState* S, SegDesc* segs
   if (t == 0) { *n_seg = 2 * nv; S->zero = 0; }
 }
 
+// ---- map outputs (:803-848)
+// segment s of a region: cube cube_of(s / 2), type s % 2 -- per cube the corner points, then the surf points (:811-812, :828-829)
+__device__ __forceinline__ int region_cube(const MapperState* S, int region, int cube_pos) { return region == ALOAM_MAP_SURROUND ? S->valid[cube_pos] : cube_pos; }
+
+// one CTA: exclusive scan of the segment sizes of `region` -> seg_off[0 .. nseg], *total = seg_off[nseg]
+__global__ void __launch_bounds__(1024) k_export_offsets(const MapperState* __restrict__ S, int region, int* __restrict__ seg_off, int* __restrict__ total) {
+  const int nseg = region == ALOAM_MAP_SURROUND ? 2 * S->n_valid : 2 * NCUBE;
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const int per = (nseg + blockDim.x - 1) / blockDim.x;
+  const int s0 = min(nseg, tid * per), s1 = min(nseg, s0 + per);
+  int sum = 0;
+  for (int s = s0; s < s1; ++s) {
+    const int ty = s & 1, slab = S->slab_of[ty][region_cube(S, region, s >> 1)];
+    sum += slab < 0 ? 0 : S->cnt[ty][slab];
+  }
+  // block-wide exclusive scan of the per-thread sums
+  int incl = sum;
+  for (int d = 1; d < 32; d <<= 1) { const int v = __shfl_up_sync(0xffffffffu, incl, d); if (lane >= d) incl += v; }
+  __shared__ int s_warp[32];
+  if (lane == 31) s_warp[warp] = incl;
+  __syncthreads();
+  if (warp == 0) {
+    int w = lane < (int)(blockDim.x >> 5) ? s_warp[lane] : 0;
+    for (int d = 1; d < 32; d <<= 1) { const int v = __shfl_up_sync(0xffffffffu, w, d); if (lane >= d) w += v; }
+    s_warp[lane] = w;
+  }
+  __syncthreads();
+  int off = incl - sum + (warp ? s_warp[warp - 1] : 0);
+  for (int s = s0; s < s1; ++s) {
+    seg_off[s] = off;
+    const int ty = s & 1, slab = S->slab_of[ty][region_cube(S, region, s >> 1)];
+    off += slab < 0 ? 0 : S->cnt[ty][slab];
+  }
+  if (tid == blockDim.x - 1) { seg_off[nseg] = off; *total = off; }
+}
+
+// one CTA per segment: the points of one (cube, type) slab to out + seg_off[s]; empty segments leave at once
+__global__ void __launch_bounds__(256) k_export_copy(const MapperState* __restrict__ S, int region, const int* __restrict__ seg_off, const Pt4* __restrict__ p0,
+                                                     const Pt4* __restrict__ p1, int cap0, int cap1, Pt4* __restrict__ out) {
+  const int s = blockIdx.x;
+  const int nseg = region == ALOAM_MAP_SURROUND ? 2 * S->n_valid : 2 * NCUBE;
+  if (s >= nseg) return;
+  const int off = seg_off[s], n = seg_off[s + 1] - off;
+  if (n == 0) return;
+  const int ty = s & 1, slab = S->slab_of[ty][region_cube(S, region, s >> 1)];
+  const Pt4* __restrict__ src = (ty ? p1 : p0) + (size_t)slab * (ty ? cap1 : cap0);
+  for (int i = threadIdx.x; i < n; i += blockDim.x) out[off + i] = src[i];
+}
+
+// /velodyne_cloud_registered (:838-848): pointAssociateToMap of a cloud with pose x7.  n = *d_n (or n_host when d_n is null);
+// the points go to out[range[0] ...] when range[1] <= capacity (range null: to out[0 .. n))
+__global__ void __launch_bounds__(256) k_associate_to_map(const Pt4* __restrict__ in, const int* __restrict__ d_n, int n_host, const long long* __restrict__ range,
+                                                          long long capacity, const double* __restrict__ x7, Pt4* __restrict__ out) {
+  const int n = d_n ? *d_n : n_host;
+  long long base = 0;
+  if (range) {
+    base = range[0];
+    if (range[1] > capacity) return;   // this scan does not fit: the caller's buffer keeps a prefix of whole scans
+  }
+  const PoseD P = load_pose(x7);
+  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) out[base + i] = point_associate_to_map(in[i], P);
+}
+
+// stage C of the registered stream: scan k's ring-major cloud to its slot buffer, and off[k + 1] = off[k] + n (off[0] = 0)
+__global__ void __launch_bounds__(256) k_stage_full(const Pt4* __restrict__ full, const int* __restrict__ d_n, int k, Pt4* __restrict__ dst, long long* __restrict__ off) {
+  const int n = *d_n;
+  if (blockIdx.x == 0 && threadIdx.x == 0) {
+    const long long base = k ? off[k] : 0;
+    if (k == 0) off[0] = 0;
+    off[k + 1] = base + n;
+  }
+  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) dst[i] = full[i];
+}
+
+int grid_for(int n) { return std::max(1, std::min((n + 255) / 256, 148 * 4)); }
+
 int ensure_mapper(aloam_ctx* c) {
   if (c->mapper) return ALOAM_OK;
   if (c->cfg.max_map_points <= 0) return ALOAM_ERR_CAPACITY;
@@ -387,6 +477,7 @@ int ensure_mapper(aloam_ctx* c) {
   ok = ok && cudaMalloc((void**)&m->d_bbox, ALOAM_MAX_SEGS * 6 * sizeof(int)) == cudaSuccess;
   ok = ok && cudaMalloc((void**)&m->d_total, 16) == cudaSuccess;
   ok = ok && cudaMalloc((void**)&m->d_pose_io, 16 * sizeof(double)) == cudaSuccess;
+  ok = ok && cudaMalloc((void**)&m->d_seg_off, (2 * NCUBE + 2) * sizeof(int)) == cudaSuccess;
   ok = ok && cudaStreamCreateWithFlags(&m->s_aux, cudaStreamNonBlocking) == cudaSuccess;
   ok = ok && cudaEventCreateWithFlags(&m->ev_fork, cudaEventDisableTiming) == cudaSuccess && cudaEventCreateWithFlags(&m->ev_join, cudaEventDisableTiming) == cudaSuccess;
   // the re-filter sorts every point of the valid cubes (<= the submap capacity per type), the stack filter two scan clouds
@@ -416,7 +507,7 @@ extern "C" void aloam_mapper_free_impl(aloam_ctx* c) {
   if (m->s_aux) { cudaStreamSynchronize(m->s_aux); cudaStreamDestroy(m->s_aux); }
   if (m->ev_fork) cudaEventDestroy(m->ev_fork);
   if (m->ev_join) cudaEventDestroy(m->ev_join);
-  void* ps[] = {m->d_world, m->d_cube, m->d_state, m->d_segs, m->d_nseg, m->d_off, m->d_rank0, m->d_bbox, m->d_total, m->d_pose_io};
+  void* ps[] = {m->d_world, m->d_cube, m->d_state, m->d_segs, m->d_nseg, m->d_off, m->d_rank0, m->d_bbox, m->d_total, m->d_pose_io, m->d_seg_off, m->d_export};
   for (void* p : ps) if (p) cudaFree(p);
   if (m->h_state) cudaFreeHost(m->h_state);
   vox_seg_free(m->buf);
@@ -483,7 +574,15 @@ int mapper_step_device(aloam_ctx* c, const Pt4* d_corner_last, const int* d_nc, 
     while (cube_bits < 31 && (double)(1ull << cube_bits) < cells) ++cube_bits; }
   vox_seg_filter(c, make_filter(m, cube_bits), m->buf, 2 * 75, (int)std::min(m->buf.cap, (size_t)2 * m->max_sub + (size_t)2 * c->max_points), m->cap[1]);
   CUDA_CHECK_RET(cudaGetLastError());
+  m->stepped = true;
   return ALOAM_OK;
+}
+
+void map_out_stage_full(aloam_ctx* c, const Pt4* full, const int* d_n, int n_upper, int k, Pt4* dst, long long* off) {
+  LAUNCH(c, KID_MAP_OUTPUT, k_stage_full, grid_for(n_upper), 256, 0, full, d_n, k, dst, off);
+}
+void map_out_register(aloam_ctx* c, const Pt4* src, const int* d_n, int n_upper, const long long* off_k, long long capacity, const double* x7, Pt4* out) {
+  LAUNCH(c, KID_MAP_OUTPUT, k_associate_to_map, grid_for(n_upper), 256, 0, src, d_n, 0, off_k, capacity, x7, out);
 }
 
 extern "C" {
@@ -503,6 +602,7 @@ int aloam_mapper_reset(aloam_ctx* c) {
   }
   CUDA_CHECK_RET(cudaMemcpyAsync(m->d_state, h, sizeof(*h), cudaMemcpyHostToDevice, c->stream));
   CUDA_CHECK_RET(cudaStreamSynchronize(c->stream));
+  m->stepped = false;
   return ALOAM_OK;
 }
 
@@ -573,6 +673,60 @@ int aloam_mapper_debug_cube(aloam_ctx* c, int which, int cube, aloam_cloud_view*
   const int n = s < 0 ? 0 : m->h_state->cnt[which][s];
   out->data = reinterpret_cast<const float*>(c->h_out[4]); out->n = n; out->stride_floats = 4;
   if (n > 0) CUDA_CHECK_RET(cudaMemcpy(c->h_out[4], m->d_pts[which] + (size_t)s * m->cap[which], (size_t)n * sizeof(Pt4), cudaMemcpyDeviceToHost));
+  return ALOAM_OK;
+}
+
+int aloam_mapper_export(aloam_ctx* c, int region, float* out, long long capacity_points, long long* n_points) {
+  if (!c || !n_points || (region != ALOAM_MAP_SURROUND && region != ALOAM_MAP_ALL) || capacity_points < 0 || (!out && capacity_points != 0))
+    return ALOAM_ERR_INVALID_ARG;
+  if (!c->mapper) return ALOAM_ERR_STATE;
+  Mapper* m = static_cast<Mapper*>(c->mapper);
+  CUDA_CHECK_RET(cudaSetDevice(c->cfg.device));
+  // sizes and offsets on the device (one scan over <= 2 x 4851 counts), one synchronisation to learn the total
+  LAUNCH(c, KID_MAP_OUTPUT, k_export_offsets, 1, 1024, 0, (const MapperState*)m->d_state, region, m->d_seg_off, m->d_seg_off + 2 * NCUBE + 1);
+  CUDA_CHECK_RET(cudaMemcpyAsync(c->h_ints + 120, m->d_seg_off + 2 * NCUBE + 1, sizeof(int), cudaMemcpyDeviceToHost, c->stream));
+  CUDA_CHECK_RET(cudaStreamSynchronize(c->stream));
+  CUDA_CHECK_RET(cudaGetLastError());
+  const long long n = c->h_ints[120];
+  *n_points = n;
+  if (!out) return ALOAM_OK;                                  // size query
+  if (n > capacity_points) return ALOAM_ERR_CAPACITY;        // nothing written
+  if (n == 0) return ALOAM_OK;
+  cudaPointerAttributes pa;
+  if (cudaPointerGetAttributes(&pa, out) != cudaSuccess) { cudaGetLastError(); pa.type = cudaMemoryTypeUnregistered; }
+  const bool on_device = pa.type == cudaMemoryTypeDevice || pa.type == cudaMemoryTypeManaged;
+  Pt4* dst = reinterpret_cast<Pt4*>(out);
+  if (!on_device) {   // host memory: through the mapper's staging buffer, then one copy
+    if (m->export_cap < (size_t)n) {
+      if (m->d_export) cudaFree(m->d_export);
+      m->d_export = nullptr; m->export_cap = 0;
+      CUDA_CHECK_RET(cudaMalloc((void**)&m->d_export, (size_t)n * sizeof(Pt4)));
+      m->export_cap = (size_t)n;
+    }
+    dst = m->d_export;
+  }
+  LAUNCH(c, KID_MAP_OUTPUT, k_export_copy, region == ALOAM_MAP_SURROUND ? 2 * kMaxValid : 2 * NCUBE, 256, 0, (const MapperState*)m->d_state, region,
+         (const int*)m->d_seg_off, (const Pt4*)m->d_pts[0], (const Pt4*)m->d_pts[1], m->cap[0], m->cap[1], dst);
+  if (!on_device) CUDA_CHECK_RET(cudaMemcpyAsync(out, dst, (size_t)n * sizeof(Pt4), cudaMemcpyDeviceToHost, c->stream));
+  CUDA_CHECK_RET(cudaStreamSynchronize(c->stream));
+  CUDA_CHECK_RET(cudaGetLastError());
+  return ALOAM_OK;
+}
+
+int aloam_mapper_associate_to_map(aloam_ctx* c, aloam_cloud_view in, float* out) {
+  if (!c || (!out && in.n > 0)) return ALOAM_ERR_INVALID_ARG;
+  int rc = check_view(in); if (rc) return rc;
+  if (in.n > c->max_points) return ALOAM_ERR_CAPACITY;
+  if (!c->mapper || !static_cast<Mapper*>(c->mapper)->stepped) return ALOAM_ERR_STATE;
+  if (in.n == 0) return ALOAM_OK;
+  Mapper* m = static_cast<Mapper*>(c->mapper);
+  CUDA_CHECK_RET(cudaSetDevice(c->cfg.device));
+  rc = upload_cloud(c, in, m->d_in[0], c->max_points); if (rc) return rc;
+  LAUNCH(c, KID_MAP_OUTPUT, k_associate_to_map, grid_for(in.n), 256, 0, (const Pt4*)m->d_in[0], (const int*)nullptr, in.n, (const long long*)nullptr, 0LL,
+         (const double*)m->d_state->x, m->d_world);
+  CUDA_CHECK_RET(cudaMemcpyAsync(out, m->d_world, (size_t)in.n * sizeof(Pt4), cudaMemcpyDefault, c->stream));
+  CUDA_CHECK_RET(cudaStreamSynchronize(c->stream));
+  CUDA_CHECK_RET(cudaGetLastError());
   return ALOAM_OK;
 }
 

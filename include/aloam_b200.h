@@ -47,6 +47,10 @@ extern "C" {
 #define ALOAM_FLAG_MAP_TOO_THIN 2
 #define ALOAM_FLAG_INITIALISED_ONLY 4 /* first frame: laserOdometry.cpp:267-271 */
 #define ALOAM_FLAG_CUBE_OVERFLOW 8    /* map cube store: a cube slab (16 k corner / 64 k surf points) or the slab pool was full; the overflow was dropped */
+#define ALOAM_FLAG_OUTPUT_TRUNCATED 16 /* aloam_scan_stream_mapped_registered: the registered clouds did not all fit the caller's buffer */
+
+#define ALOAM_MAP_SURROUND 0 /* aloam_mapper_export: the valid cubes of the last frame, laserCloudSurroundInd (laserMapping.cpp:806-814) */
+#define ALOAM_MAP_ALL 1      /* aloam_mapper_export: all 21 x 21 x 11 cubes in index order (laserMapping.cpp:823-830) */
 
 typedef struct aloam_ctx aloam_ctx;
 
@@ -212,6 +216,29 @@ int aloam_mapper_step(aloam_ctx* ctx, aloam_cloud_view corner_last, aloam_cloud_
 int aloam_mapper_debug_state(aloam_ctx* ctx, int centre[3], int* n_valid, int valid[125], double q_wmap_wodom[4],
                              double t_wmap_wodom[3], long long totals[2]);
 int aloam_mapper_debug_cube(aloam_ctx* ctx, int which, int cube_index, aloam_cloud_view* out);
+
+/* ---- map outputs: the three clouds alaserMapping publishes at the end of a frame (laserMapping.cpp:803-848).  Outputs are
+ * packed stride-4 points in caller-owned memory (a map has no fixed upper size, so there is no ctx-owned output view).
+ * aloam_mapper_export: /laser_cloud_surround (region ALOAM_MAP_SURROUND, published by the reference every 5th frame) or
+ * /laser_cloud_map (ALOAM_MAP_ALL, every 20th frame) -- per cube the corner points, then the surf points, in the reference's
+ * order; the store as it is after the last frame's insertion and per-cube VoxelGrid.  Publish cadence is the caller's choice.
+ * out == NULL with capacity_points == 0 is a size query.  A result larger than capacity_points returns ALOAM_ERR_CAPACITY with
+ * the required size in *n_points and writes nothing.  out may be host (pageable or pinned) or device memory.
+ * ALOAM_ERR_STATE before the mapper exists; 0 points after aloam_mapper_reset.
+ * aloam_mapper_associate_to_map: /velodyne_cloud_registered -- pointAssociateToMap (:154-163) of a whole cloud (the full-
+ * resolution /velodyne_cloud_3) with the refined pose of the last frame; the intensity is kept.  in: stride 4 or 8, host or
+ * device, n <= cfg.max_points; out: in.n points, host or device.  ALOAM_ERR_STATE before the first frame since a reset.
+ * aloam_scan_stream_mapped_registered: aloam_scan_stream_mapped, and every scan's ring-major full cloud (what /velodyne_cloud_2
+ * and, unchanged, /velodyne_cloud_3 carry) registered with the scan's refined pose and written to registered[offsets[k] ...].
+ * offsets (n_scans + 1) are the prefix sums of the cloud sizes and are always filled.  Scans that end beyond capacity_points
+ * are not written (the buffer holds a prefix of whole scans) and ALOAM_FLAG_OUTPUT_TRUNCATED is set in stats_last->flags;
+ * the poses are complete either way.  registered must be device memory or page-locked host memory (written by a kernel);
+ * pageable memory is ALOAM_ERR_INVALID_ARG, reported before any work is issued. */
+int aloam_mapper_export(aloam_ctx* ctx, int region, float* out, long long capacity_points, long long* n_points);
+int aloam_mapper_associate_to_map(aloam_ctx* ctx, aloam_cloud_view in, float* out);
+int aloam_scan_stream_mapped_registered(aloam_ctx* ctx, const aloam_cloud_view* raws, int n_scans, int device_resident,
+                                        double* odom_poses, double* map_poses, float* registered, long long capacity_points,
+                                        long long* offsets, aloam_stats* stats_last);
 
 /* ---- multi-GPU scan-to-map (one process per GPU).  Rank 0 creates the 128-byte id and ships it to the others;
  * after aloam_comm_init each rank uploads only ITS shard of the submap (x-slabs of aloam_shard_slab_cells() cells of
